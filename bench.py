@@ -7,7 +7,8 @@
 A "step" is one pass of the hot path over one batch: StableDiffusion::sample_image for `--batch` images
 (20 DDIM steps x (cond+uncond UNet) + VAE decode + u8 pack). Default workload = BASELINE configs[1]
 (batch 1, 512x512, 20 steps, cfg 7.5) on every rank (weak scaling: per-GPU work is fixed).
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0. With --dump-outputs DIR, the images the last timed step produced are written to DIR as
+float32 .npy (same arguments -> same inputs, so two builds can be compared output for output).
 """
 import argparse
 import json
@@ -20,6 +21,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ from this process
+
+DUMP_BUDGET_BYTES = 64 << 20  # all files of one --dump-outputs directory together
 
 METRIC = "images_per_sec_512x512_20steps"
 UNIT = "images/s"
@@ -174,6 +178,18 @@ def gpu_eager_times():
                     "a labelled secondary comparator, not the reference and not this repo's path"}
 
 
+def dump_outputs(out_dir, name, a, budget_bytes):
+    """Writes `a` as out_dir/<name>.npy in float32; above `budget_bytes`, a fixed seeded sample of its flattened values instead,
+    as out_dir/<name>_sample.npy (the same positions for the same shape, so samples of two runs compare element for element)."""
+    import numpy as np
+    a = np.ascontiguousarray(a, np.float32)
+    if a.nbytes > budget_bytes:
+        keep = np.sort(np.random.default_rng(0).choice(a.size, budget_bytes // 4, replace=False))
+        a, name = a.reshape(-1)[keep], name + "_sample"
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """Reference arm: the reference's own implementation cannot be built here (Rust, no toolchain; DESIGN.md §2), so this times
     the CPU port of the same path on the host cores. A bench "step" of this arm is ONE real DDIM step of the workload (2 UNet
@@ -224,7 +240,14 @@ def main():
     ap.add_argument("--no-c5", action="store_true", help="multi-GPU runs: skip the BASELINE configs[4] sub-record (8 images per rank)")
     ap.add_argument("--ref-cuda", action="store_true",
                     help="with --impl reference: also time the torch restatement on cuda:0 (labelled secondary comparator)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the u8 images of the last timed step as float32 DIR/images.npy (images_rank<r>.npy per rank "
+                         "with several GPUs; a seeded sample when above 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to this repo's CUDA path")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -289,10 +312,10 @@ def main():
             # the public host-buffer call: H2D of context/uncond/latent, sampling, D2H of the u8 images — all inside
             ctx.check(ctx.lib.sdb_sample_image(ctx.h, _lib.ptr(p_ctx.numpy()), n, L, _lib.ptr(p_unc.numpy()), Lu, 7.5, args.ddim_steps,
                                                _lib.ptr(p_lat.numpy()), 0, Hl, Hl, p_rgb.numpy().ctypes.data_as(_lib._u8p)))
-        return dev_step, e2e_step, int(h_ctx.nbytes + h_unc.nbytes + h_lat.nbytes), int(p_rgb.numel())
+        return dev_step, e2e_step, int(h_ctx.nbytes + h_unc.nbytes + h_lat.nbytes), int(p_rgb.numel()), d_rgb
 
     n = args.batch
-    step_dev, step_e2e, h2d, d2h = make_steps(n)
+    step_dev, step_e2e, h2d, d2h, d_rgb = make_steps(n)
 
     def barrier():
         torch.cuda.synchronize()
@@ -327,6 +350,9 @@ def main():
     launches = ctx.launch_count() - l0
     clocks = sampler.window(w0, w1) if rank == 0 else None
     value = world * n * args.steps / (ms * 1e-3)
+    if args.dump_outputs:  # d_rgb holds what the last timed step wrote; nothing has run since
+        dump_outputs(args.dump_outputs, "images" if world == 1 else f"images_rank{rank}", d_rgb.cpu().numpy(),
+                     DUMP_BUDGET_BYTES // world)
 
     # ---- end to end through the host-buffer C ABI
     step_e2e()
@@ -343,7 +369,7 @@ def main():
     # the same call with 8 images per rank (world * 8 images per step), its own clocks sample; the headline stays configs[1]
     c5 = None
     if world > 1 and args.batch != 8 and not args.no_c5:
-        c5_dev, c5_e2e, c5_h2d, c5_d2h = make_steps(8)
+        c5_dev, c5_e2e, c5_h2d, c5_d2h, _ = make_steps(8)
         for _ in range(2):
             c5_dev()
         k5 = max(2, min(args.steps, 5))

@@ -1,7 +1,7 @@
-"""Generates tests/golden/ref_python.npz: outputs of the REFERENCE'S OWN Python model (/root/reference/python/dump.py, run
-unmodified on tests/ref_shim/tinygrad) on this repo's synthetic weights (seed 0). Needs /root/reference (this container only).
+"""Generates tests/golden/ref_python.npz: outputs of the REFERENCE'S OWN Python model (<reference checkout>/python/dump.py, run
+unmodified on tests/ref_shim/tinygrad) on this repo's synthetic weights (seed 0). Needs a checkout of the reference.
 
-  python tests/ref_shim/make_ref_golden.py
+  python tests/ref_shim/make_ref_golden.py <reference checkout>
 
 How the synthetic weights get into the reference model: the reference's saver (python/stablediffusion.py:8-14) writes the
 randomly initialised model as a dump-dir; every file it wrote is matched back to the parameter it came from, which yields the
@@ -10,6 +10,7 @@ dump-dir name (and orientation) of every parameter; the synthetic tensors are th
 import os
 import shutil
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -41,12 +42,13 @@ def inputs():
 def main():
     torch.set_num_threads(os.cpu_count())
     t0 = time.time()
-    ref = R.Reference(seed=0)
-    tmp = "/dev/shm/sdb200_ref_dump" if os.path.isdir("/dev/shm") else "/tmp/sdb200_ref_dump"
-    shutil.rmtree(tmp, ignore_errors=True)
-    ref.save(tmp)
-    ref.derive_names(tmp)
-    shutil.rmtree(tmp, ignore_errors=True)
+    ref = R.Reference(sys.argv[1], seed=0)
+    tmp = tempfile.mkdtemp(prefix="sdb200_ref_dump")
+    try:
+        ref.save(tmp)
+        ref.derive_names(tmp)
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
     print("reference model built, saved by its own saver, names derived:", len(ref.names), f"{time.time() - t0:.0f}s", flush=True)
     n = ref.assign(synth.make_params(0))
     assert n == len(ref.names), (n, len(ref.names))

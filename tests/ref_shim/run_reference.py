@@ -1,4 +1,4 @@
-"""Runs the reference's own Python model (/root/reference/python/dump.py, imported unmodified) on the tinygrad stand-in.
+"""Runs the reference's own Python model (<reference checkout>/python/dump.py, imported unmodified) on the tinygrad stand-in.
 
 TEST INFRASTRUCTURE. What is reference-authored here: the model topology and op sequence (python/dump.py:24-350, 352-461),
 the savers that define the dump-dir names, transposes and metadata the Rust loaders read (python/save.py, unet.py,
@@ -7,6 +7,7 @@ autoencoder.py, clip.py, stablediffusion.py). What is not: the primitive tensor 
 from __future__ import annotations
 
 import contextlib
+import hashlib
 import io
 import os
 import sys
@@ -14,18 +15,16 @@ import sys
 import numpy as np
 import torch
 
-REF_PY = "/root/reference/python"
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 
 
-def available() -> bool:
-    return os.path.isfile(os.path.join(REF_PY, "dump.py"))
-
-
-def load_dump_module():
-    """import /root/reference/python/dump.py with the stand-in `tinygrad` package ahead of everything else."""
-    for p in (HERE, REF_PY):
+def load_dump_module(ref_dir: str):
+    """import <ref_dir>/python/dump.py with the stand-in `tinygrad` package ahead of everything else."""
+    ref_py = os.path.join(ref_dir, "python")
+    if not os.path.isfile(os.path.join(ref_py, "dump.py")):
+        raise FileNotFoundError(f"{ref_py}/dump.py: not a checkout of the reference")
+    for p in (HERE, ref_py):
         if p not in sys.path:
             sys.path.insert(0, p)
     if ROOT not in sys.path:
@@ -53,6 +52,24 @@ def _params_of(obj, seen, out):
             _params_of(o, seen, out)
 
 
+SMALL_FILE = 8192  # dump-dir files up to this size are compared by value, larger ones by size
+
+
+def tree_manifest(root: str) -> dict:
+    """relative path -> [size, digest of the stored values (files up to SMALL_FILE bytes) or None] for every file under `root`."""
+    out = {}
+    for d, _, fs in os.walk(root):
+        for f in fs:
+            p = os.path.join(d, f)
+            size = os.path.getsize(p)
+            digest = None
+            if size <= SMALL_FILE:
+                a = np.load(p)
+                digest = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()[:16]
+            out[os.path.relpath(p, root)] = [size, digest]
+    return out
+
+
 def _fingerprint(a: np.ndarray):
     f = np.ascontiguousarray(a, np.float32).reshape(-1)
     return (tuple(a.shape), f[:6].tobytes(), f[-6:].tobytes())
@@ -62,8 +79,8 @@ class Reference:
     """The reference StableDiffusion object (python/dump.py:565-570) with random stand-in weights, plus the dump-dir name of
     every parameter, DERIVED by running the reference's own saver and matching what it wrote against the parameters."""
 
-    def __init__(self, seed: int = 0, verbose: bool = False):
-        self.dump = load_dump_module()
+    def __init__(self, ref_dir: str, seed: int = 0, verbose: bool = False):
+        self.dump = load_dump_module(ref_dir)
         from tinygrad import nn
         from tinygrad.tensor import Tensor
         self.Tensor = Tensor

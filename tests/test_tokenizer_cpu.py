@@ -1,21 +1,28 @@
-"""The reference's only test, reproduced (src/tokenizer.rs:205-221): the one golden vector the reference holds."""
+"""The reference's only test, reproduced (src/tokenizer.rs:205-221): the one golden vector the reference holds.
+
+The merge table is the part of the reference's bpe_simple_vocab_16e6.txt the tokenizer reads (header + 48894 merges), stored
+xz-compressed under tests/golden (tests/ref_shim/make_ref_fixtures.py)."""
+import lzma
 import os
 
 import pytest
 
 from stable_diffusion_burn_b200 import tokenizer as T
 
-try:
-    VOCAB = T.find_vocab()
-except FileNotFoundError:
-    VOCAB = None
-
-pytestmark = pytest.mark.skipif(VOCAB is None, reason="bpe_simple_vocab_16e6.txt (reference data file) not available")
+VOCAB_XZ = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", T.VOCAB_FILE + ".xz")
 
 
 @pytest.fixture(scope="module")
-def tok():
-    return T.SimpleTokenizer(VOCAB)
+def vocab(tmp_path_factory):
+    path = tmp_path_factory.mktemp("bpe") / T.VOCAB_FILE
+    with lzma.open(VOCAB_XZ, "rt", encoding="utf-8") as f:
+        path.write_text(f.read(), encoding="utf-8")
+    return str(path)
+
+
+@pytest.fixture(scope="module")
+def tok(vocab):
+    return T.SimpleTokenizer(vocab)
 
 
 def test_reference_kat_encode_decode(tok):
@@ -41,12 +48,12 @@ def test_cleaning_quirks(tok):
     assert tok.decode(tok.encode("café ☕")).strip() == "café ☕"
 
 
-def test_agrees_with_an_independent_clip_tokenizer(tok, tmp_path):
+def test_agrees_with_an_independent_clip_tokenizer(tok, vocab, tmp_path):
     """Second opinion on the mirror: transformers.CLIPTokenizer (independently written from the same published BPE) built from the
     same merges file must produce the same ids on plain prompts (no ftfy-specific cleaning involved)."""
     tr = pytest.importorskip("transformers")
     import json
-    merges = open(VOCAB, encoding="utf-8").read().split("\n")[1:49152 - 256 - 2 + 1]
+    merges = open(vocab, encoding="utf-8").read().split("\n")[1:49152 - 256 - 2 + 1]
     vocab = [u for _, u in T._byte_unicode_table()]
     vocab = vocab + [v + "</w>" for v in vocab] + ["".join(m.split()) for m in merges] + ["<|startoftext|>", "<|endoftext|>"]
     (tmp_path / "vocab.json").write_text(json.dumps({v: i for i, v in enumerate(vocab)}))
