@@ -56,7 +56,8 @@ int sdb_get_tensor(sdb_ctx* ctx, const char* name, float* host, int64_t count);
  * src/model/load.rs:17-47; <path>/<tensor name>.npy, the schedule from <path>/alphas_cumprod.npy). Optional files follow
  * the reference (missing Linear/Conv bias = none, missing GroupNorm weight/bias = ones/zeros); the configuration scalars
  * the reference reads (eps, n_group, stride, padding, n_head, n_layer, n_steps ...) are validated against the compiled
- * SD-v1.4 topology and each norm's eps is honoured. Encoder / quant_conv files are not read (not on the path). */
+ * SD-v1.4 topology and each norm's eps is honoured. The encoder / quant_conv files are read too (sdb_encode_image and
+ * sdb_img2img use them). */
 int sdb_load_dump_dir(sdb_ctx* ctx, const char* path);
 /* load_tensor::<B, D> (src/model/load.rs:30-47) for one file, no context needed: splits the leading `ndim` shape values
  * from the data. Returns the element count (data may be NULL to probe), or -1 (text via sdb_last_error(NULL)). */
@@ -118,9 +119,29 @@ int sdb_clip_forward_dev(sdb_ctx* ctx, const int32_t* d_tokens, int n, int L, fl
 
 /* ---- VAE encoder (SURVEY §8f row f4) ---------------------------------------------------------------- */
 /* Autoencoder::encode_image (src/model/autoencoder/mod.rs:60-66): img [n,3,H,W] -> latent [n,4,H/8,W/8] = the first four
- * channels of quant_conv(encoder(img)). H, W multiples of 8 (>= 64). Only img2img needs it; the reference CLI never calls it. */
+ * channels of quant_conv(encoder(img)). H, W multiples of 8 (>= 64). sdb_img2img builds on it; the reference CLI never calls it. */
 int sdb_encode_image(sdb_ctx* ctx, const float* img, int n, int H, int W, float* latent);
 int sdb_encode_image_dev(sdb_ctx* ctx, const float* d_img, int n, int H, int W, float* d_latent, void* stream);
+
+/* ---- img2img and inpainting (DESIGN.md §7 row f5) ------------------------------------------------------- */
+/* The reference has no img2img; this is SDEdit / latent-blend inpainting on its schedule and sampler
+ * (src/model/stablediffusion/mod.rs:102-160). H, W are latent sizes as in sdb_sample_image.
+ *  rgb [n,8H,8W,3] u8 (the layout sdb_sample_image writes) -> x = rgb * fl32(2/255) - 1 -> x0 = 0.18215 * encode_image(x).
+ *  Of the T timesteps of the n_steps schedule the last n_run = min(T, floor(strength * T + 1e-9)) run, starting from
+ *  sqrt(a[t0]) x0 + sqrt(1 - a[t0]) noise; strength 0 returns x0 with no UNet pass. noise [n,4,H,W], or NULL for the N(0,1)
+ *  stream keyed by `seed` that sdb_sample_latent draws its initial latent from.
+ *  mask [n,8H,8W] u8 or NULL: nonzero = repaint. A latent cell is repainted if any pixel of its 8x8 block is; after every
+ *  step the other cells are reset to the known image noised to the step's target timestep (x0 itself after the last step),
+ *  and rgb_out pixels whose mask is 0 are copied from rgb. The SD-v1.4 UNet has 4 input channels: no 9-channel inpainting.
+ *  latent_out [n,4,H,W] and rgb_out [n,8H,8W,3] may each be NULL, but not both. Errors: strength NaN or outside [0,1],
+ *  rgb NULL, n_steps outside [1,1000], sizes the encoder or the UNet reject. */
+int sdb_img2img(sdb_ctx* ctx, const uint8_t* rgb, const uint8_t* mask, const float* context, int n, int L,
+                const float* uncond, int Lu, double guidance_scale, int n_steps, double strength,
+                const float* noise, uint64_t seed, int H, int W, float* latent_out, uint8_t* rgb_out);
+int sdb_img2img_dev(sdb_ctx* ctx, const uint8_t* d_rgb, const uint8_t* d_mask, const float* d_context, int n, int L,
+                    const float* d_uncond, int Lu, double guidance_scale, int n_steps, double strength,
+                    const float* d_noise, uint64_t seed, int H, int W, float* d_latent_out, uint8_t* d_rgb_out,
+                    void* stream);
 
 /* ---- hot path, device buffers (zero-copy callers) ------------------------------------------ */
 int sdb_unet_forward_dev(sdb_ctx* ctx, const float* d_x, int32_t timestep, const float* d_context,

@@ -44,6 +44,14 @@ extern "C" {
     fn sdb_forward_diffuser(ctx: *mut SdbCtx, latent: *const f32, timestep: i32, context: *const f32, n: c_int, l: c_int,
                             uncond: *const f32, lu: c_int, guidance_scale: f64, h: c_int, w: c_int, pred: *mut f32,
                             out_uncond: *mut f32, out_cond: *mut f32) -> c_int;
+    fn sdb_img2img(ctx: *mut SdbCtx, rgb: *const u8, mask: *const u8, context: *const f32, n: c_int, l: c_int,
+                   uncond: *const f32, lu: c_int, guidance_scale: f64, n_steps: c_int, strength: f64, noise: *const f32,
+                   seed: u64, h: c_int, w: c_int, latent_out: *mut f32, rgb_out: *mut u8) -> c_int;
+    #[allow(dead_code)]
+    fn sdb_img2img_dev(ctx: *mut SdbCtx, d_rgb: *const c_void, d_mask: *const c_void, d_context: *const c_void, n: c_int,
+                       l: c_int, d_uncond: *const c_void, lu: c_int, guidance_scale: f64, n_steps: c_int, strength: f64,
+                       d_noise: *const c_void, seed: u64, h: c_int, w: c_int, d_latent_out: *mut c_void,
+                       d_rgb_out: *mut c_void, stream: *mut c_void) -> c_int;
     fn sdb_nccl_unique_id(id128: *mut c_void) -> c_int;
     fn sdb_broadcast_weights(ctx: *mut SdbCtx, id128: *const c_void, rank: c_int, world: c_int) -> c_int;
     #[allow(dead_code)]
@@ -178,6 +186,23 @@ impl StableDiffusion {
                                  pred.as_mut_ptr(), std::ptr::null_mut(), std::ptr::null_mut())
         })?;
         Ok(pred)
+    }
+
+    /// img2img (SDEdit) and, with `mask`, latent-blend inpainting on the sample_latent sampler (DESIGN.md §7 row f5; the reference
+    /// has no img2img). `rgb` is [n, 8h, 8w, 3] u8 like the images sample_image returns, `mask` [n, 8h, 8w] (nonzero = repaint),
+    /// `strength` in [0, 1] the share of the n_steps schedule that runs, `noise = None` draws N(0,1) on the device from `seed`.
+    #[allow(clippy::too_many_arguments)]
+    pub fn img2img(&self, rgb: &[u8], [n, h, w]: [usize; 3], mask: Option<&[u8]>, context: &[f32], l: usize,
+                   unconditional_context: &[f32], lu: usize, unconditional_guidance_scale: f64, n_steps: usize, strength: f64,
+                   noise: Option<&[f32]>, seed: u64) -> Result<Vec<Vec<u8>>, SdbError> {
+        let mut out = vec![0u8; n * 8 * h * 8 * w * 3];
+        self.check(unsafe {
+            sdb_img2img(self.ctx, rgb.as_ptr(), mask.map_or(std::ptr::null(), |s| s.as_ptr()), context.as_ptr(), n as c_int,
+                        l as c_int, unconditional_context.as_ptr(), lu as c_int, unconditional_guidance_scale, n_steps as c_int,
+                        strength, noise.map_or(std::ptr::null(), |s| s.as_ptr()), seed, h as c_int, w as c_int,
+                        std::ptr::null_mut(), out.as_mut_ptr())
+        })?;
+        Ok(out.chunks(8 * h * 8 * w * 3).map(|c| c.to_vec()).collect())
     }
 
     /// Multi-GPU init: rank 0 calls `nccl_unique_id()` and ships the 128 bytes to the other ranks by any means; every rank then

@@ -50,6 +50,11 @@ SIGNATURES = [
     ("sdb_read_dump_tensor", C.c_int64, [C.c_char_p, C.c_int, C.POINTER(C.c_int64), _f32p, C.c_int64]),
     ("sdb_encode_image", C.c_int, [_ctx, _f32p, C.c_int, C.c_int, C.c_int, _f32p]),
     ("sdb_encode_image_dev", C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    ("sdb_img2img", C.c_int, [_ctx, _u8p, _u8p, _f32p, C.c_int, C.c_int, _f32p, C.c_int, C.c_double, C.c_int, C.c_double,
+                              _f32p, C.c_uint64, C.c_int, C.c_int, _f32p, _u8p]),
+    ("sdb_img2img_dev", C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_double,
+                                  C.c_int, C.c_double, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                  C.c_void_p]),
     ("sdb_clip_forward", C.c_int, [_ctx, C.POINTER(C.c_int32), C.c_int, C.c_int, _f32p]),
     ("sdb_clip_forward_dev", C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     ("sdb_unet_forward_dev", C.c_int, [_ctx, C.c_void_p, C.c_int32, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -256,6 +261,33 @@ class Context:
                                              ptr(init_latent) if init_latent is not None else None, seed, H, W,
                                              rgb.ctypes.data_as(_u8p)))
         return rgb
+
+    def img2img(self, context, uncond, scale, n_steps, rgb, strength, mask=None, noise=None, seed=0, latent=True, image=True):
+        """rgb [n,8H,8W,3] u8, mask [n,8H,8W] (nonzero = repaint) or None, noise [n,4,H,W] or None (seeded stream).
+        -> (latent [n,4,H,W] or None, rgb [n,8H,8W,3] u8 or None); `latent` / `image` select the outputs."""
+        context = f32(context); uncond = f32(uncond)
+        rgb = np.ascontiguousarray(rgb, dtype=np.uint8)
+        n, L, _ = context.shape
+        if rgb.ndim != 4 or rgb.shape[0] != n or rgb.shape[3] != 3:
+            raise ValueError(f"rgb must be [n={n}, 8H, 8W, 3] uint8, got {rgb.shape}")
+        H, W = rgb.shape[1] // 8, rgb.shape[2] // 8
+        if rgb.shape[1] != 8 * H or rgb.shape[2] != 8 * W:
+            raise ValueError(f"image height and width must be multiples of 8, got {rgb.shape[1:3]}")
+        if mask is not None:
+            mask = np.ascontiguousarray(mask, dtype=np.uint8)
+            if mask.shape != rgb.shape[:3]:
+                raise ValueError(f"mask must be [n, 8H, 8W] = {rgb.shape[:3]}, got {mask.shape}")
+        if noise is not None:
+            noise = f32(noise)
+            if noise.shape != (n, 4, H, W):
+                raise ValueError(f"noise must be [n, 4, H, W] = {(n, 4, H, W)}, got {noise.shape}")
+        lat = np.empty((n, 4, H, W), np.float32) if latent else None
+        out = np.empty_like(rgb) if image else None
+        self.check(self.lib.sdb_img2img(self.h, rgb.ctypes.data_as(_u8p), mask.ctypes.data_as(_u8p) if mask is not None else None,
+                                        ptr(context), n, L, ptr(uncond), uncond.shape[0], float(scale), int(n_steps),
+                                        float(strength), ptr(noise) if noise is not None else None, int(seed), H, W,
+                                        ptr(lat) if lat is not None else None, out.ctypes.data_as(_u8p) if out is not None else None))
+        return lat, out
 
     # ---- profiling
     def profile(self, on=True):

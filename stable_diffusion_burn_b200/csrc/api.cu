@@ -380,6 +380,27 @@ int sdb_encode_image_dev(sdb_ctx* ctx, const float* d_img, int n, int H, int W, 
   API_END
 }
 
+int sdb_img2img(sdb_ctx* ctx, const uint8_t* rgb, const uint8_t* mask, const float* context, int n, int L, const float* uncond,
+                int Lu, double guidance_scale, int n_steps, double strength, const float* noise, uint64_t seed, int H, int W,
+                float* latent_out, uint8_t* rgb_out) {
+  API_BEGIN(ctx)
+  need_final(c);
+  SDB_CHECK(context && uncond, "null argument");
+  model_img2img_host(c, rgb, mask, context, n, L, uncond, Lu, guidance_scale, n_steps, strength, noise, seed, H, W, latent_out,
+                     rgb_out);
+  API_END
+}
+
+int sdb_img2img_dev(sdb_ctx* ctx, const uint8_t* d_rgb, const uint8_t* d_mask, const float* d_context, int n, int L,
+                    const float* d_uncond, int Lu, double guidance_scale, int n_steps, double strength, const float* d_noise,
+                    uint64_t seed, int H, int W, float* d_latent_out, uint8_t* d_rgb_out, void* stream) {
+  API_BEGIN(ctx)
+  need_final(c);
+  model_img2img_dev(c, d_rgb, d_mask, d_context, n, L, d_uncond, Lu, guidance_scale, n_steps, strength, d_noise, seed, H, W,
+                    d_latent_out, d_rgb_out, (cudaStream_t)stream);
+  API_END
+}
+
 int sdb_clip_forward(sdb_ctx* ctx, const int32_t* tokens, int n, int L, float* out) {
   API_BEGIN(ctx)
   need_final(c);

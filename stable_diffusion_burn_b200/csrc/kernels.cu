@@ -1128,6 +1128,133 @@ void to_rgb8_launch(const float* img_nchw, int n, int H, int W, uint8_t* rgb, cu
   SDB_CUDA(cudaGetLastError());
 }
 
+// ============================================================ img2img / inpainting (DESIGN.md §7 row f5)
+// u8 HWC [n][H][W][3] -> fp32 planes [n][4][H][W] (fourth plane zero, the layout of the encoder's Cin = 4 conv_in):
+// x = fl(fl(v * fl32(2/255)) - 1), no FMA, so numpy fp32 reproduces it bit for bit
+__global__ void rgb8_to_planes4_kernel(const uint8_t* __restrict__ rgb, int HW, long long total, float* __restrict__ img4) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int p = int(i % HW);
+    const long long r = i / HW;
+    const int c = int(r % 4);
+    const long long n = r / 4;
+    img4[i] = c < 3 ? __fsub_rn(__fmul_rn((float)rgb[(n * HW + p) * 3 + c], (float)(2.0 / 255.0)), 1.0f) : 0.0f;
+  }
+}
+void rgb8_to_planes4_launch(const uint8_t* rgb, int n, int H, int W, float* img4, cudaStream_t st) {
+  const long long total = (long long)n * 4 * H * W;
+  int grid = (int)((total + 255) / 256);
+  if (grid > 148 * 16) grid = 148 * 16;
+  rgb8_to_planes4_kernel<<<grid, 256, 0, st>>>(rgb, H * W, total, img4);
+  SDB_CUDA(cudaGetLastError());
+}
+
+// latent cell (y, x) is repainted when any pixel of its 8x8 block is: m[n][H][W] = max over the block of (mask != 0)
+__global__ void latent_mask_kernel(const uint8_t* __restrict__ mask, int H, int W, long long total, uint8_t* __restrict__ m) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int x = int(i % W);
+    const long long r = i / W;
+    const int y = int(r % H);
+    const long long n = r / H;
+    const uint8_t* blk = mask + ((n * 8 * H + 8 * y) * 8 * W + 8 * x);
+    uint32_t any = 0;
+#pragma unroll
+    for (int dy = 0; dy < 8; ++dy)
+#pragma unroll
+      for (int dx = 0; dx < 8; ++dx) any |= blk[(size_t)dy * 8 * W + dx];
+    m[i] = any ? 1 : 0;
+  }
+}
+void latent_mask_launch(const uint8_t* mask, int n, int H, int W, uint8_t* m, cudaStream_t st) {
+  const long long total = (long long)n * H * W;
+  int grid = (int)((total + 255) / 256);
+  if (grid > 148 * 8) grid = 148 * 8;
+  latent_mask_kernel<<<grid, 256, 0, st>>>(mask, H, W, total, m);
+  SDB_CUDA(cudaGetLastError());
+}
+
+__global__ void scale_kernel(float* __restrict__ x, long long count, float s) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x)
+    x[i] = __fmul_rn(x[i], s);
+}
+void scale_launch(float* x, long long count, float s, cudaStream_t st) {
+  int grid = (int)((count + 255) / 256);
+  if (grid > 148 * 8) grid = 148 * 8;
+  scale_kernel<<<grid, 256, 0, st>>>(x, count, s);
+  SDB_CUDA(cudaGetLastError());
+}
+
+// x_t0 = fl(fl(a * x0) + fl(b * eps)) into both halves of the batch-2n UNet input (as cfg_ddim_kernel writes them)
+__global__ void noise_latent_kernel(const float* __restrict__ x0, const float* __restrict__ eps, long long count, float a, float b,
+                                    float* __restrict__ lat) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x) {
+    const float v = __fadd_rn(__fmul_rn(a, x0[i]), __fmul_rn(b, eps[i]));
+    lat[i] = v;
+    lat[i + count] = v;
+  }
+}
+void noise_latent_launch(const float* x0, const float* eps, long long count, float a, float b, float* latent, cudaStream_t st) {
+  int grid = (int)((count + 255) / 256);
+  if (grid > 148 * 8) grid = 148 * 8;
+  noise_latent_kernel<<<grid, 256, 0, st>>>(x0, eps, count, a, b, latent);
+  SDB_CUDA(cudaGetLastError());
+}
+
+// cfg_ddim_kernel's update, then the kept cells (m == 0) are selected from the known image noised to a_prev:
+// known = fl(fl(sqrt(a_prev) * x0) + fl(sqrt(1 - a_prev) * eps)) — the same two coefficients as the update's
+__global__ void cfg_ddim_blend_kernel(const float* __restrict__ eu, const float* __restrict__ ec, float* __restrict__ lat,
+                                      long long count, float scale, float sqrt_1m_at, float sqrt_at, float sqrt_aprev,
+                                      float dir_coef, const float* __restrict__ x0, const float* __restrict__ eps,
+                                      const uint8_t* __restrict__ m, int HW) {
+  pdl_enter();
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x) {
+    const float u = eu[i], c = ec[i];
+    const float pred = u + (c - u) * scale;               // stablediffusion/mod.rs:190-191
+    const float px0 = (lat[i] - pred * sqrt_1m_at) / sqrt_at;  // :152
+    float nl = px0 * sqrt_aprev + pred * dir_coef;        // :153-155 (sigma = 0)
+    const long long cell = (i / (4LL * HW)) * HW + i % HW;
+    if (!m[cell]) nl = __fadd_rn(__fmul_rn(sqrt_aprev, x0[i]), __fmul_rn(dir_coef, eps[i]));
+    lat[i] = nl;
+    lat[i + count] = nl;
+  }
+}
+void cfg_ddim_blend_launch(const float* eps_u, const float* eps_c, float* latent, long long count, float scale,
+                           float sqrt_one_minus_at, float sqrt_at, float sqrt_aprev, float dir_coef, const float* x0,
+                           const float* eps, const uint8_t* m, int HW, cudaStream_t st) {
+  int grid = (int)((count + 255) / 256);
+  if (grid > 148 * 8) grid = 148 * 8;
+  launch_k(cfg_ddim_blend_kernel, dim3(grid), dim3(256), 0, st, eps_u, eps_c, latent, count, scale, sqrt_one_minus_at, sqrt_at,
+           sqrt_aprev, dir_coef, x0, eps, m, HW);
+  SDB_CUDA(cudaGetLastError());
+}
+
+// to_rgb8_kernel's conversion, except that pixels with mask == 0 are copied from the source image unchanged
+__global__ void to_rgb8_paste_kernel(const float* __restrict__ img, int HW, long long total, const uint8_t* __restrict__ src,
+                                     const uint8_t* __restrict__ mask, uint8_t* __restrict__ rgb) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = i / 3;
+    if (!mask[r]) {
+      rgb[i] = src[i];
+      continue;
+    }
+    const int c = int(i % 3);
+    const int p = int(r % HW);
+    const long long n = r / HW;
+    float v = img[(n * 3 + c) * HW + p];
+    v = (v + 1.0f) / 2.0f * 255.0f;             // stablediffusion/mod.rs:79-84
+    float mm = (v != v) ? 255.0f : fminf(v, 255.0f);
+    mm = fmaxf(mm, 0.0f);
+    rgb[i] = (uint8_t)mm;
+  }
+}
+void to_rgb8_paste_launch(const float* img_nchw, int n, int H, int W, const uint8_t* src_rgb, const uint8_t* mask, uint8_t* rgb,
+                          cudaStream_t st) {
+  const long long total = (long long)n * 3 * H * W;
+  int grid = (int)((total + 255) / 256);
+  if (grid > 148 * 16) grid = 148 * 16;
+  to_rgb8_paste_kernel<<<grid, 256, 0, st>>>(img_nchw, H * W, total, src_rgb, mask, rgb);
+  SDB_CUDA(cudaGetLastError());
+}
+
 
 __device__ __forceinline__ uint32_t mix32(uint32_t x) {
   x ^= x >> 16;

@@ -99,6 +99,22 @@ void cfg_ddim_launch(const float* eps_u, const float* eps_c, float* latent, long
 void cfg_combine_launch(const float* eps_u, const float* eps_c, long long count, float scale, float* pred, cudaStream_t st);
 // u8 = trunc(clamp((img+1)/2*255, 0, 255)), NCHW fp32 -> NHWC u8 (reference stablediffusion/mod.rs:79-97)
 void to_rgb8_launch(const float* img_nchw, int n, int H, int W, uint8_t* rgb, cudaStream_t st);
+// ---- img2img / inpainting (DESIGN.md §7 row f5)
+// u8 HWC [n][H][W][3] -> fp32 NCHW [n][4][H][W] with a zero fourth plane: x = fl(fl(v * fl32(2/255)) - 1), no FMA
+void rgb8_to_planes4_launch(const uint8_t* rgb, int n, int H, int W, float* img4, cudaStream_t st);
+// pixel mask [n][8H][8W] (nonzero = repaint) -> latent mask [n][H][W] in {0,1}: max over each 8x8 block
+void latent_mask_launch(const uint8_t* mask, int n, int H, int W, uint8_t* m, cudaStream_t st);
+// x = fl(x * s) in place
+void scale_launch(float* x, long long count, float s, cudaStream_t st);
+// x_t0 = fl(fl(a*x0) + fl(b*eps)), written to both halves of latent [2*count] (uncond | cond inputs)
+void noise_latent_launch(const float* x0, const float* eps, long long count, float a, float b, float* latent, cudaStream_t st);
+// cfg_ddim_launch, then cells with m[n][HW] == 0 take fl(fl(sqrt_aprev*x0) + fl(dir_coef*eps)); latent [n][4][HW] twice
+void cfg_ddim_blend_launch(const float* eps_u, const float* eps_c, float* latent, long long count, float scale,
+                           float sqrt_one_minus_at, float sqrt_at, float sqrt_aprev, float dir_coef, const float* x0,
+                           const float* eps, const uint8_t* m, int HW, cudaStream_t st);
+// to_rgb8_launch where pixels with mask[n][H][W] == 0 are copied from src_rgb [n][H][W][3]
+void to_rgb8_paste_launch(const float* img_nchw, int n, int H, int W, const uint8_t* src_rgb, const uint8_t* mask, uint8_t* rgb,
+                          cudaStream_t st);
 void quant_conv_slice_launch(const float* x, const float* w, const float* b, int n, int HW, float* y, cudaStream_t st);
 void add_vec_launch(const float* a, const float* b, int n, float* y, cudaStream_t st);
 // N(0,1) latents from a Philox-like counter hash (used only when the caller passes no init latent)

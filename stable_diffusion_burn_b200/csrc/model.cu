@@ -1004,9 +1004,13 @@ void model_decode_host(Ctx& c, const float* latent, int n, int H, int W, float* 
   SDB_CUDA(cudaStreamSynchronize(c.stream));
 }
 
-void model_encode_dev(Ctx& c, const float* d_img, int n, int H, int W, float* d_latent, cudaStream_t caller) {
+static void check_encode_size(int n, int H, int W) {
   SDB_CHECK(n >= 1 && H >= 64 && W >= 64 && H % 8 == 0 && W % 8 == 0 && ((H / 8) * (W / 8)) % 8 == 0,
             "encode_image: height and width must be multiples of 8, at least 64, with (H/8)*(W/8) a multiple of 8");
+}
+
+void model_encode_dev(Ctx& c, const float* d_img, int n, int H, int W, float* d_latent, cudaStream_t caller) {
+  check_encode_size(n, H, W);
   StreamJoin join(c, caller);
   c.work.reset();
   const size_t plane = (size_t)H * W;
@@ -1033,13 +1037,18 @@ void model_encode_host(Ctx& c, const float* img, int n, int H, int W, float* lat
   SDB_CUDA(cudaStreamSynchronize(c.stream));
 }
 
-// latent_to_image (stablediffusion/mod.rs:69-100)
-static void latent_to_image_dev(Ctx& c, const float* d_latent, int n, int H, int W, uint8_t* d_rgb) {
+// latent_to_image (stablediffusion/mod.rs:69-100). With a pixel mask [n,8H,8W], pixels whose mask is 0 are copied from
+// paste_rgb [n,8H,8W,3] instead (inpainting keeps the known image byte for byte).
+static void latent_to_image_dev(Ctx& c, const float* d_latent, int n, int H, int W, uint8_t* d_rgb,
+                                const uint8_t* paste_rgb = nullptr, const uint8_t* paste_mask = nullptr) {
   float* d_img = c.work.get<float>((size_t)n * 3 * 64 * H * W);
   // `latent * (1.0 / 0.18215)`: the scalar is rounded to f32 before the multiply, as burn's mul_scalar does
   decode_chunked(c, d_latent, n, H, W, (float)(1.0 / 0.18215), d_img);
   KernelScope ks(c, KC_ELEMENTWISE);
-  to_rgb8_launch(d_img, n, 8 * H, 8 * W, d_rgb, c.stream);
+  if (paste_mask)
+    to_rgb8_paste_launch(d_img, n, 8 * H, 8 * W, paste_rgb, paste_mask, d_rgb, c.stream);
+  else
+    to_rgb8_launch(d_img, n, 8 * H, 8 * W, d_rgb, c.stream);
 }
 
 void model_latent_to_image_host(Ctx& c, const float* latent, int n, int H, int W, uint8_t* rgb) {
@@ -1053,17 +1062,34 @@ void model_latent_to_image_host(Ctx& c, const float* latent, int n, int H, int W
   SDB_CUDA(cudaStreamSynchronize(c.stream));
 }
 
-// sample_latent + latent_to_image (stablediffusion/mod.rs:51-160). The conditional and unconditional UNet
-// evaluations of a step (forward_diffuser :162-192) run as ONE batch-2n pass: weights stream from HBM once.
-void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale,
-                      int n_steps, const float* d_init_latent, int H, int W, float* d_latent_out, uint8_t* d_rgb,
-                      cudaStream_t caller) {
-  Model& m = M(c);
+static void check_sample_args(int n, int L, int Lu, int n_steps, int H, int W) {
   SDB_CHECK(n >= 1 && L >= 1 && Lu >= 1, "sample arguments");
   SDB_CHECK(n_steps >= 1 && n_steps <= 1000, "n_steps must be in [1,1000] (step_by(0) panics in the reference)");
   SDB_CHECK(H % 8 == 0 && W % 8 == 0, "latent size must be a multiple of 8");
   SDB_CHECK(((H / 8) * (W / 8)) % 8 == 0, "unsupported latent size: (H/8)*(W/8) must be a multiple of 8");
-  StreamJoin join(c, caller);
+}
+
+// timesteps (stablediffusion/mod.rs:111,123): (0..1000).rev().step_by(1000 / n_steps)
+static std::vector<int> ddim_timesteps(int n_steps) {
+  std::vector<int> ts;
+  for (int t = 999; t >= 0; t -= 1000 / n_steps) ts.push_back(t);
+  return ts;
+}
+
+// Where a sampler run starts and what it blends (img2img / inpainting, DESIGN.md §7 row f5). The default is text-to-image.
+struct SampleStart {
+  int i0 = 0;                  // index of the first timestep of ddim_timesteps(n_steps) that runs
+  const float* x0 = nullptr;   // [n,4,H,W] encoded image: the start latent is fl(fl(a*x0) + fl(b*eps)) at ts[i0]
+  const float* eps = nullptr;  // [n,4,H,W] noise of the start latent and of the kept cells
+  const uint8_t* m = nullptr;  // [n,H,W] latent mask (0 = keep the known image) or null: no blend
+};
+
+// The DDIM / CFG loop of sample_latent over ts[st.i0:]. Leaves the final latent in the first half of the batch-2n input it
+// returns, with the work arena at the mark after the step state, so the caller can decode from there. The work-arena layout
+// depends on (n, L, Lu, H, W) only: every start index and blend state replays the same cached step graph.
+static float* sample_loop(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale,
+                          int n_steps, const float* d_init_latent, const SampleStart& st, int H, int W) {
+  Model& m = M(c);
   c.work.reset();
   const int nb = 2 * n;
   const int Lpad = round_up(std::max(L, Lu), 32);
@@ -1079,12 +1105,19 @@ void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float*
     SDB_CUDA(cudaMemcpyAsync(ctxp + (size_t)i * Lpad * 768, d_uncond, (size_t)Lu * 768 * 4, cudaMemcpyDeviceToDevice, c.stream));
   SDB_CUDA(cudaMemcpy2DAsync(ctxp + (size_t)n * Lpad * 768, (size_t)Lpad * 768 * 4, d_context, (size_t)L * 768 * 4,
                              (size_t)L * 768 * 4, n, cudaMemcpyDeviceToDevice, c.stream));
-  SDB_CUDA(cudaMemcpyAsync(xb, d_init_latent, le * 4, cudaMemcpyDeviceToDevice, c.stream));
-  SDB_CUDA(cudaMemcpyAsync(xb + le, d_init_latent, le * 4, cudaMemcpyDeviceToDevice, c.stream));
-  // timesteps (stablediffusion/mod.rs:111,123): (0..1000).rev().step_by(1000 / n_steps)
   const int step = 1000 / n_steps;
-  std::vector<int> ts;
-  for (int t = 999; t >= 0; t -= step) ts.push_back(t);
+  std::vector<int> ts = ddim_timesteps(n_steps);
+  SDB_CHECK(st.i0 >= 0 && st.i0 < (int)ts.size(), "sampler start index");
+  ts.erase(ts.begin(), ts.begin() + st.i0);
+  if (st.x0) {
+    // x_t0 = sqrt(a[t0]) x0 + sqrt(1 - a[t0]) eps with the coefficients widened to f64 like the DDIM update's
+    const double a0 = (double)m.alphas_host[ts[0]];
+    KernelScope ks(c, KC_ELEMENTWISE);
+    noise_latent_launch(st.x0, st.eps, (long long)le, (float)std::sqrt(a0), (float)std::sqrt(1.0 - a0), xb, c.stream);
+  } else {
+    SDB_CUDA(cudaMemcpyAsync(xb, d_init_latent, le * 4, cudaMemcpyDeviceToDevice, c.stream));
+    SDB_CUDA(cudaMemcpyAsync(xb + le, d_init_latent, le * 4, cudaMemcpyDeviceToDevice, c.stream));
+  }
   std::vector<int> lens(nb);
   for (int i = 0; i < nb; ++i) lens[i] = i < n ? Lu : L;
   SDB_CUDA(cudaMemcpyAsync(d_t, ts.data(), ts.size() * 4, cudaMemcpyHostToDevice, c.stream));
@@ -1122,9 +1155,11 @@ void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float*
   cudaGraphExec_t exec = nullptr;
   int64_t graph_launches = 0;
   if (use_graph) {
+    // the graph bakes in every work-arena address allocated after work_mark: a layout change must never replay it
     for (auto& g : m.graphs)
-      if (g.key == key && g.io[0] == (void*)xb && g.io[1] == (void*)eps && g.io[2] == (void*)cs.kv[0].kv) exec = g.exec,
-          graph_launches = (int64_t)(intptr_t)g.io[3];
+      if (g.key == key && g.io[0] == (void*)xb && g.io[1] == (void*)eps && g.io[2] == (void*)cs.kv[0].kv &&
+          g.io[4] == (void*)(uintptr_t)work_mark)
+        exec = g.exec, graph_launches = (int64_t)(intptr_t)g.io[3];
     if (!exec) {
       // warm-up pass outside capture (sets kernel attributes), then capture
       SDB_CUDA(cudaMemcpyAsync(d_tcur, d_t, 4, cudaMemcpyDeviceToDevice, c.stream));
@@ -1149,6 +1184,7 @@ void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float*
       ge.key = key, ge.exec = exec;
       memset(ge.io, 0, sizeof(ge.io));
       ge.io[0] = xb, ge.io[1] = eps, ge.io[2] = cs.kv[0].kv, ge.io[3] = (void*)(intptr_t)graph_launches;
+      ge.io[4] = (void*)(uintptr_t)work_mark;
       m.graphs.push_back(ge);
     }
   }
@@ -1166,12 +1202,119 @@ void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float*
       unet_pass(c, nb, xb, d_tcur, nullptr, Lpad, d_len, H, W, eps, &cs, emb_all);
     }
     KernelScope ks(c, KC_ELEMENTWISE);
-    cfg_ddim_launch(eps, eps + le, xb, (long long)le, (float)scale, (float)std::sqrt(1.0 - a_t), (float)std::sqrt(a_t),
-                    (float)std::sqrt(a_prev), (float)std::sqrt(1.0 - a_prev), c.stream);
+    if (st.m)
+      cfg_ddim_blend_launch(eps, eps + le, xb, (long long)le, (float)scale, (float)std::sqrt(1.0 - a_t), (float)std::sqrt(a_t),
+                            (float)std::sqrt(a_prev), (float)std::sqrt(1.0 - a_prev), st.x0, st.eps, st.m, H * W, c.stream);
+    else
+      cfg_ddim_launch(eps, eps + le, xb, (long long)le, (float)scale, (float)std::sqrt(1.0 - a_t), (float)std::sqrt(a_t),
+                      (float)std::sqrt(a_prev), (float)std::sqrt(1.0 - a_prev), c.stream);
   }
   c.work.off = work_mark;
+  return xb;
+}
+
+// sample_latent + latent_to_image (stablediffusion/mod.rs:51-160). The conditional and unconditional UNet
+// evaluations of a step (forward_diffuser :162-192) run as ONE batch-2n pass: weights stream from HBM once.
+void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale,
+                      int n_steps, const float* d_init_latent, int H, int W, float* d_latent_out, uint8_t* d_rgb,
+                      cudaStream_t caller) {
+  check_sample_args(n, L, Lu, n_steps, H, W);
+  StreamJoin join(c, caller);
+  float* xb = sample_loop(c, d_context, n, L, d_uncond, Lu, scale, n_steps, d_init_latent, SampleStart{}, H, W);
+  const size_t le = (size_t)n * 4 * H * W;
   if (d_latent_out) SDB_CUDA(cudaMemcpyAsync(d_latent_out, xb, le * 4, cudaMemcpyDeviceToDevice, c.stream));
   if (d_rgb) latent_to_image_dev(c, xb, n, H, W, d_rgb);
+}
+
+// ---- img2img (SDEdit) and latent-blend inpainting (DESIGN.md §7 row f5). The reference has no img2img: this is the standard
+// construction on its own schedule and sampler (oracle/img2img_oracle.py states it once).
+static void check_img2img_args(const uint8_t* rgb, const void* latent_out, const void* rgb_out, int n, int L, int Lu,
+                               int n_steps, double strength, int H, int W) {
+  SDB_CHECK(rgb, "img2img: rgb is null");
+  SDB_CHECK(latent_out || rgb_out, "img2img: latent_out and rgb_out are both null");
+  SDB_CHECK(strength >= 0.0 && strength <= 1.0, "img2img: strength must lie in [0, 1]");  // false for NaN
+  check_sample_args(n, L, Lu, n_steps, H, W);
+  check_encode_size(n, 8 * H, 8 * W);
+}
+
+// schedule index of the first step that runs: n_run = min(T, floor(strength * T + 1e-9)) of the T steps run, from T - n_run
+static int img2img_start_index(int n_steps, double strength) {
+  const int T = (int)ddim_timesteps(n_steps).size();
+  return T - std::min(T, (int)std::floor(strength * T + 1e-9));
+}
+
+void model_img2img_dev(Ctx& c, const uint8_t* d_rgb_in, const uint8_t* d_mask, const float* d_context, int n, int L,
+                       const float* d_uncond, int Lu, double scale, int n_steps, double strength, const float* d_noise,
+                       uint64_t seed, int H, int W, float* d_latent_out, uint8_t* d_rgb, cudaStream_t caller) {
+  check_img2img_args(d_rgb_in, d_latent_out, d_rgb, n, L, Lu, n_steps, strength, H, W);
+  StreamJoin join(c, caller);
+  const size_t le = (size_t)n * 4 * H * W;
+  // x0, eps and the latent mask outlive the work-arena reset of the step loop: Ctx::state, not the work arena
+  float* x0 = (float*)c.state(0, le * 4);
+  const float* eps = d_noise;
+  if (!d_noise) {
+    float* e = (float*)c.state(1, le * 4);
+    KernelScope ks(c, KC_ELEMENTWISE);
+    randn_launch(e, (long long)le, seed, c.stream);  // the stream text-to-image draws its initial latent from
+    eps = e;
+  }
+  uint8_t* lm = nullptr;
+  if (d_mask) {
+    lm = (uint8_t*)c.state(2, (size_t)n * H * W);
+    KernelScope ks(c, KC_ELEMENTWISE);
+    latent_mask_launch(d_mask, n, H, W, lm, c.stream);
+  }
+  // x0 = fl(encode_image(rgb * fl32(2/255) - 1) * 0.18215f), the inverse of latent_to_image's latent * (1 / 0.18215)
+  c.work.reset();
+  const size_t plane = (size_t)64 * H * W;
+  for (int i0 = 0; i0 < n; i0 += 4) {  // chunks of 4 images, as model_encode_dev
+    const int nb = std::min(4, n - i0);
+    const size_t mark = c.work.off;
+    float* img4 = c.work.get<float>((size_t)nb * 4 * plane);
+    {
+      KernelScope ks(c, KC_ELEMENTWISE);
+      rgb8_to_planes4_launch(d_rgb_in + (size_t)i0 * 3 * plane, nb, 8 * H, 8 * W, img4, c.stream);
+    }
+    Fwd f(c, nb);
+    vae_encode(f, img4, 8 * H, 8 * W, x0 + (size_t)i0 * 4 * H * W);
+    c.work.off = mark;
+  }
+  {
+    KernelScope ks(c, KC_ELEMENTWISE);
+    scale_launch(x0, (long long)le, 0.18215f, c.stream);
+  }
+  const int i0 = img2img_start_index(n_steps, strength);
+  const float* lat = x0;  // strength 0: nothing runs, the result is x0
+  if (i0 < (int)ddim_timesteps(n_steps).size()) {
+    SampleStart st;
+    st.i0 = i0, st.x0 = x0, st.eps = eps, st.m = lm;
+    lat = sample_loop(c, d_context, n, L, d_uncond, Lu, scale, n_steps, nullptr, st, H, W);
+  }
+  if (d_latent_out) SDB_CUDA(cudaMemcpyAsync(d_latent_out, lat, le * 4, cudaMemcpyDeviceToDevice, c.stream));
+  if (d_rgb) latent_to_image_dev(c, lat, n, H, W, d_rgb, d_rgb_in, d_mask);
+}
+
+void model_img2img_host(Ctx& c, const uint8_t* rgb_in, const uint8_t* mask, const float* context, int n, int L,
+                        const float* uncond, int Lu, double scale, int n_steps, double strength, const float* noise, uint64_t seed,
+                        int H, int W, float* latent_out, uint8_t* rgb) {
+  check_img2img_args(rgb_in, latent_out, rgb, n, L, Lu, n_steps, strength, H, W);
+  const size_t le = (size_t)n * 4 * H * W, ce = (size_t)n * L * 768, ue = (size_t)Lu * 768, re = (size_t)n * 3 * 64 * H * W;
+  uint8_t* d_in = (uint8_t*)c.io(0, re);
+  uint8_t* d_m = mask ? (uint8_t*)c.io(1, (size_t)n * 64 * H * W) : nullptr;
+  float* d_c = (float*)c.io(2, ce * 4);
+  float* d_u = (float*)c.io(3, ue * 4);
+  float* d_n = noise ? (float*)c.io(4, le * 4) : nullptr;
+  float* d_lo = latent_out ? (float*)c.io(5, le * 4) : nullptr;
+  uint8_t* d_r = rgb ? (uint8_t*)c.io(6, re) : nullptr;
+  SDB_CUDA(cudaMemcpyAsync(d_in, rgb_in, re, cudaMemcpyHostToDevice, c.stream));
+  if (mask) SDB_CUDA(cudaMemcpyAsync(d_m, mask, (size_t)n * 64 * H * W, cudaMemcpyHostToDevice, c.stream));
+  SDB_CUDA(cudaMemcpyAsync(d_c, context, ce * 4, cudaMemcpyHostToDevice, c.stream));
+  SDB_CUDA(cudaMemcpyAsync(d_u, uncond, ue * 4, cudaMemcpyHostToDevice, c.stream));
+  if (noise) SDB_CUDA(cudaMemcpyAsync(d_n, noise, le * 4, cudaMemcpyHostToDevice, c.stream));
+  model_img2img_dev(c, d_in, d_m, d_c, n, L, d_u, Lu, scale, n_steps, strength, d_n, seed, H, W, d_lo, d_r, c.stream);
+  if (latent_out) SDB_CUDA(cudaMemcpyAsync(latent_out, d_lo, le * 4, cudaMemcpyDeviceToHost, c.stream));
+  if (rgb) SDB_CUDA(cudaMemcpyAsync(rgb, d_r, re, cudaMemcpyDeviceToHost, c.stream));
+  SDB_CUDA(cudaStreamSynchronize(c.stream));
 }
 
 void model_sample_host(Ctx& c, const float* context, int n, int L, const float* uncond, int Lu, double scale, int n_steps,

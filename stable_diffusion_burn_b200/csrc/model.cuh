@@ -23,6 +23,14 @@ void model_sample_host(Ctx& c, const float* context, int n, int L, const float* 
 void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale,
                       int n_steps, const float* d_init_latent, int H, int W, float* d_latent_out, uint8_t* d_rgb,
                       cudaStream_t caller);
+// img2img / latent-blend inpainting on the DDIM sampler: rgb [n,8H,8W,3] u8, optional pixel mask [n,8H,8W] (nonzero =
+// repaint), optional noise [n,4,H,W] (else randn_launch keyed by seed); latent_out / rgb_out may each be null, not both
+void model_img2img_dev(Ctx& c, const uint8_t* d_rgb_in, const uint8_t* d_mask, const float* d_context, int n, int L,
+                       const float* d_uncond, int Lu, double scale, int n_steps, double strength, const float* d_noise,
+                       uint64_t seed, int H, int W, float* d_latent_out, uint8_t* d_rgb, cudaStream_t caller);
+void model_img2img_host(Ctx& c, const uint8_t* rgb_in, const uint8_t* mask, const float* context, int n, int L,
+                        const float* uncond, int Lu, double scale, int n_steps, double strength, const float* noise, uint64_t seed,
+                        int H, int W, float* latent_out, uint8_t* rgb);
 void model_forward_diffuser_dev(Ctx& c, const float* d_latent, int t, const float* d_context, int n, int L, const float* d_uncond,
                                 int Lu, double scale, int H, int W, float* d_pred, float* d_u, float* d_c, cudaStream_t caller);
 void model_forward_diffuser_host(Ctx& c, const float* latent, int t, const float* context, int n, int L, const float* uncond,

@@ -38,8 +38,7 @@ void* Arena::alloc(size_t bytes) {
   return base + a;
 }
 
-void* Ctx::io(int slot, size_t bytes) {
-  IoBuf& b = iobuf[slot];
+static void* grow(Ctx::IoBuf& b, size_t bytes, cudaStream_t stream) {
   if (bytes > b.cap) {
     SDB_CUDA(cudaStreamSynchronize(stream));  // nothing queued may still read the old buffer
     if (b.p) cudaFree(b.p);
@@ -50,11 +49,15 @@ void* Ctx::io(int slot, size_t bytes) {
   }
   return b.p;
 }
+void* Ctx::io(int slot, size_t bytes) { return grow(iobuf[slot], bytes, stream); }
+void* Ctx::state(int slot, size_t bytes) { return grow(statebuf[slot], bytes, stream); }
 void Ctx::io_destroy() {
-  for (IoBuf& b : iobuf) {
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr, b.cap = 0;
-  }
+  for (IoBuf* set : {iobuf, statebuf})
+    for (int i = 0; i < 8; ++i) {
+      IoBuf& b = set[i];
+      if (b.p) cudaFree(b.p);
+      b.p = nullptr, b.cap = 0;
+    }
 }
 
 float* Ctx::master_ptr(const std::string& name) {

@@ -147,9 +147,13 @@ struct Ctx {
   struct IoBuf {
     void* p = nullptr;
     size_t cap = 0;
-  } iobuf[6];
+  } iobuf[8];
   void* io(int slot, size_t bytes);
-  void io_destroy();
+  // grow-only device state of the img2img sampler (encoded image, noise, latent mask): it must survive the work-arena reset
+  // between the encoder and the step loop, and it is never one of the host wrappers' staging slots
+  IoBuf statebuf[8];
+  void* state(int slot, size_t bytes);
+  void io_destroy();  // frees iobuf and statebuf
   void* model = nullptr;  // Model* (model.cu)
   unsigned int* splitk_tickets = nullptr;  // 64K zeroed counters (gemm_tc split-K tile tickets)
   // SDB_DEBUG_SYNC=1: synchronise after every launch and report the failing op (bring-up aid)

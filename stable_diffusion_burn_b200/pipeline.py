@@ -106,6 +106,16 @@ class StableDiffusion:
         return self.ctx.sample_latent(context, unconditional_context, unconditional_guidance_scale, n_steps,
                                       init_latent=init_latent, seed=seed, H=height // 8, W=width // 8)
 
+    def img2img(self, context, unconditional_context, unconditional_guidance_scale: float, n_steps: int, image, strength: float,
+                mask=None, noise=None, seed: int = 0):
+        """img2img (SDEdit) and, with `mask`, latent-blend inpainting on the same DDIM sampler (DESIGN.md §7 row f5; the reference
+        has no img2img). image [n,H,W,3] uint8 (H, W multiples of 64, the layout sample_image returns), strength in [0,1] (the
+        share of the n_steps schedule that runs), mask [n,H,W] (nonzero = repaint) or None, noise [n,4,H/8,W/8] or None (the
+        seeded stream sample_image draws from). -> list of n flat uint8 arrays of H*W*3, like sample_image."""
+        _, rgb = self.ctx.img2img(context, unconditional_context, unconditional_guidance_scale, n_steps, image, strength,
+                                  mask=mask, noise=noise, seed=seed, latent=False)
+        return [rgb[i].reshape(-1) for i in range(rgb.shape[0])]
+
     def latent_to_image(self, latent):
         rgb = self.ctx.latent_to_image(latent)
         return [rgb[i].reshape(-1) for i in range(rgb.shape[0])]
