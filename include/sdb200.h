@@ -143,6 +143,32 @@ int sdb_img2img_dev(sdb_ctx* ctx, const uint8_t* d_rgb, const uint8_t* d_mask, c
                     const float* d_noise, uint64_t seed, int H, int W, float* d_latent_out, uint8_t* d_rgb_out,
                     void* stream);
 
+/* ---- selectable samplers (DESIGN.md §7 row f6) ----------------------------------------------------------- */
+/* The reference's only sampler is DDIM with sigma fixed to 0 (src/model/stablediffusion/mod.rs:119; the noise term at :155
+ * never runs). sdb_sample_ex runs sample_latent's loop (:102-160) with a selectable update on the same schedule
+ * (ts = (0..1000).rev().step_by(1000 / n_steps), T = len(ts), a_next = 1 after the last step):
+ *  SDB_SAMPLER_DDIM, eta in [0,1]: x' = x0 sqrt(a_next) + pred sqrt(1 - a_next - sigma^2) + sigma z_i with
+ *    sigma = eta sqrt((1 - a_next)/(1 - a_t)) sqrt(1 - a_t/a_next) (0 at the last step). eta = 0 is sdb_sample_latent exactly.
+ *  SDB_SAMPLER_DPMPP_2M (eta = 0): DPM-Solver++(2M), data prediction; first order at step 0, second order after it, and the
+ *    last step returns its x0 prediction.
+ * step_noise [T][n,4,H,W]: z_i is slice i; the last slice must be present but is never read (sigma = 0 there). Given only for
+ * DDIM with eta > 0. NULL: slice i is sdb_randn(seed_i, n*4*H*W) with seed_i = seed ^ ((i+1) * 0x9E3779B97F4A7C15) mod 2^64,
+ * drawn inside the update kernel. init_latent NULL: sdb_randn(seed, n*4*H*W), as sdb_sample_latent.
+ * latent_out [n,4,H,W] and rgb_out [n,8H,8W,3] may each be NULL, but not both. Errors: unknown sampler, eta NaN or outside
+ * [0,1], eta != 0 with DPM-Solver++(2M), step_noise with any other sampler than DDIM at eta > 0, and what sdb_sample_latent
+ * rejects. The time-embedding hoist and the cached step graph of sdb_sample_latent are used unchanged. */
+#define SDB_SAMPLER_DDIM 0     /* eta >= 0; eta = 0 is sdb_sample_latent exactly */
+#define SDB_SAMPLER_DPMPP_2M 1
+int sdb_sample_ex(sdb_ctx* ctx, const float* context, int n, int L, const float* uncond, int Lu, double guidance_scale,
+                  int n_steps, int sampler, double eta, const float* init_latent, const float* step_noise, uint64_t seed,
+                  int H, int W, float* latent_out, uint8_t* rgb_out);
+int sdb_sample_ex_dev(sdb_ctx* ctx, const float* d_context, int n, int L, const float* d_uncond, int Lu, double guidance_scale,
+                      int n_steps, int sampler, double eta, const float* d_init_latent, const float* d_step_noise, uint64_t seed,
+                      int H, int W, float* d_latent_out, uint8_t* d_rgb_out, void* stream);
+/* The library's seeded N(0,1) stream (the initial latent of sdb_sample_latent / sdb_sample_ex and the step noise above):
+ * count values into host memory. */
+int sdb_randn(sdb_ctx* ctx, uint64_t seed, int64_t count, float* out);
+
 /* ---- hot path, device buffers (zero-copy callers) ------------------------------------------ */
 int sdb_unet_forward_dev(sdb_ctx* ctx, const float* d_x, int32_t timestep, const float* d_context,
                          int n, int H, int W, int L, float* d_out, void* stream);

@@ -22,6 +22,17 @@ pub struct SdbCtx {
     _private: [u8; 0],
 }
 
+/// The update rule of `StableDiffusion::sample_ex` (SDB_SAMPLER_* in include/sdb200.h). `Ddim { eta: 0.0 }` is the reference's.
+#[derive(Clone, Copy, Debug)]
+pub enum Sampler {
+    /// DDIM with `eta` in [0, 1] (the `sigma` of src/model/stablediffusion/mod.rs:119, scaled by eta).
+    Ddim { eta: f64 },
+    /// DPM-Solver++(2M), data prediction, multistep.
+    DpmPp2M,
+}
+const SDB_SAMPLER_DDIM: c_int = 0;
+const SDB_SAMPLER_DPMPP_2M: c_int = 1;
+
 extern "C" {
     fn sdb_create(device: c_int, out: *mut *mut SdbCtx) -> c_int;
     fn sdb_destroy(ctx: *mut SdbCtx) -> c_int;
@@ -52,6 +63,16 @@ extern "C" {
                        l: c_int, d_uncond: *const c_void, lu: c_int, guidance_scale: f64, n_steps: c_int, strength: f64,
                        d_noise: *const c_void, seed: u64, h: c_int, w: c_int, d_latent_out: *mut c_void,
                        d_rgb_out: *mut c_void, stream: *mut c_void) -> c_int;
+    fn sdb_sample_ex(ctx: *mut SdbCtx, context: *const f32, n: c_int, l: c_int, uncond: *const f32, lu: c_int,
+                     guidance_scale: f64, n_steps: c_int, sampler: c_int, eta: f64, init_latent: *const f32,
+                     step_noise: *const f32, seed: u64, h: c_int, w: c_int, latent_out: *mut f32, rgb_out: *mut u8) -> c_int;
+    #[allow(dead_code)]
+    fn sdb_sample_ex_dev(ctx: *mut SdbCtx, d_context: *const c_void, n: c_int, l: c_int, d_uncond: *const c_void, lu: c_int,
+                         guidance_scale: f64, n_steps: c_int, sampler: c_int, eta: f64, d_init_latent: *const c_void,
+                         d_step_noise: *const c_void, seed: u64, h: c_int, w: c_int, d_latent_out: *mut c_void,
+                         d_rgb_out: *mut c_void, stream: *mut c_void) -> c_int;
+    #[allow(dead_code)]
+    fn sdb_randn(ctx: *mut SdbCtx, seed: u64, count: i64, out: *mut f32) -> c_int;
     fn sdb_nccl_unique_id(id128: *mut c_void) -> c_int;
     fn sdb_broadcast_weights(ctx: *mut SdbCtx, id128: *const c_void, rank: c_int, world: c_int) -> c_int;
     #[allow(dead_code)]
@@ -203,6 +224,28 @@ impl StableDiffusion {
                         std::ptr::null_mut(), out.as_mut_ptr())
         })?;
         Ok(out.chunks(8 * h * 8 * w * 3).map(|c| c.to_vec()).collect())
+    }
+
+    /// `sample_image` with a selectable sampler (DESIGN.md §7 row f6; the reference's only sampler is `Sampler::Ddim { eta: 0.0 }`,
+    /// src/model/stablediffusion/mod.rs:119). `step_noise` ([T, n, 4, 64, 64], DDIM with eta > 0 only) or `None`: step i draws
+    /// from the device stream keyed by `seed ^ ((i + 1) * 0x9E3779B97F4A7C15)`.
+    #[allow(clippy::too_many_arguments)]
+    pub fn sample_ex(&self, context: &[f32], [n, l]: [usize; 2], unconditional_context: &[f32], lu: usize,
+                     unconditional_guidance_scale: f64, n_steps: usize, sampler: Sampler, init_latent: Option<&[f32]>,
+                     step_noise: Option<&[f32]>, seed: u64) -> Result<Vec<Vec<u8>>, SdbError> {
+        let (h, w) = (64usize, 64usize);
+        let (id, eta) = match sampler {
+            Sampler::Ddim { eta } => (SDB_SAMPLER_DDIM, eta),
+            Sampler::DpmPp2M => (SDB_SAMPLER_DPMPP_2M, 0.0),
+        };
+        let mut rgb = vec![0u8; n * 8 * h * 8 * w * 3];
+        self.check(unsafe {
+            sdb_sample_ex(self.ctx, context.as_ptr(), n as c_int, l as c_int, unconditional_context.as_ptr(), lu as c_int,
+                          unconditional_guidance_scale, n_steps as c_int, id, eta,
+                          init_latent.map_or(std::ptr::null(), |s| s.as_ptr()), step_noise.map_or(std::ptr::null(), |s| s.as_ptr()),
+                          seed, h as c_int, w as c_int, std::ptr::null_mut(), rgb.as_mut_ptr())
+        })?;
+        Ok(rgb.chunks(8 * h * 8 * w * 3).map(|c| c.to_vec()).collect())
     }
 
     /// Multi-GPU init: rank 0 calls `nccl_unique_id()` and ships the 128 bytes to the other ranks by any means; every rank then

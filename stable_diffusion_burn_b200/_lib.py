@@ -55,6 +55,12 @@ SIGNATURES = [
     ("sdb_img2img_dev", C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_double,
                                   C.c_int, C.c_double, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                   C.c_void_p]),
+    ("sdb_sample_ex", C.c_int, [_ctx, _f32p, C.c_int, C.c_int, _f32p, C.c_int, C.c_double, C.c_int, C.c_int, C.c_double, _f32p,
+                                _f32p, C.c_uint64, C.c_int, C.c_int, _f32p, _u8p]),
+    ("sdb_sample_ex_dev", C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_double, C.c_int, C.c_int,
+                                    C.c_double, C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                    C.c_void_p]),
+    ("sdb_randn", C.c_int, [_ctx, C.c_uint64, C.c_int64, _f32p]),
     ("sdb_clip_forward", C.c_int, [_ctx, C.POINTER(C.c_int32), C.c_int, C.c_int, _f32p]),
     ("sdb_clip_forward_dev", C.c_int, [_ctx, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     ("sdb_unet_forward_dev", C.c_int, [_ctx, C.c_void_p, C.c_int32, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -81,6 +87,9 @@ SIGNATURES = [
     ("sdb_test_layernorm", C.c_int, [_ctx, _f32p, _f32p, _f32p, C.c_int, C.c_int, _f32p]),
     ("sdb_test_attention", C.c_int, [_ctx, _f32p, _f32p, _f32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _f32p]),
 ]
+
+# sampler ids of sdb_sample_ex (SDB_SAMPLER_* in include/sdb200.h)
+SAMPLERS = {"ddim": 0, "dpmpp_2m": 1}
 
 _lib = None
 
@@ -261,6 +270,38 @@ class Context:
                                              ptr(init_latent) if init_latent is not None else None, seed, H, W,
                                              rgb.ctypes.data_as(_u8p)))
         return rgb
+
+    def sample_ex(self, context, uncond, scale, n_steps, sampler="ddim", eta=0.0, init_latent=None, step_noise=None, seed=0,
+                  H=64, W=64, latent=True, image=False):
+        """Text-to-image with a selectable sampler (sdb_sample_ex): sampler "ddim" (eta in [0,1]) or "dpmpp_2m" (eta 0).
+        step_noise [T,n,4,H,W] (DDIM with eta > 0) or None (the seeded stream). -> (latent [n,4,H,W] or None, rgb
+        [n,8H,8W,3] u8 or None); `latent` / `image` select the outputs."""
+        context = f32(context); uncond = f32(uncond)
+        n, L, _ = context.shape
+        if isinstance(sampler, str) and sampler not in SAMPLERS:
+            raise ValueError(f"sampler must be one of {sorted(SAMPLERS)}, got {sampler!r}")
+        sid = SAMPLERS[sampler] if isinstance(sampler, str) else int(sampler)  # an int id goes to the library as is
+        if init_latent is not None:
+            init_latent = f32(init_latent)
+            H, W = init_latent.shape[2:]
+        if step_noise is not None:
+            step_noise = f32(step_noise)
+            T = len(range(999, -1, -(1000 // int(n_steps)))) if 1 <= int(n_steps) <= 1000 else 0
+            if step_noise.shape != (T, n, 4, H, W):
+                raise ValueError(f"step_noise must be [T, n, 4, H, W] = {(T, n, 4, H, W)}, got {step_noise.shape}")
+        lat = np.empty((n, 4, H, W), np.float32) if latent else None
+        rgb = np.empty((n, 8 * H, 8 * W, 3), np.uint8) if image else None
+        opt = lambda a: ptr(a) if a is not None else None
+        self.check(self.lib.sdb_sample_ex(self.h, ptr(context), n, L, ptr(uncond), uncond.shape[0], float(scale), int(n_steps),
+                                          sid, float(eta), opt(init_latent), opt(step_noise), int(seed), H, W,
+                                          opt(lat), rgb.ctypes.data_as(_u8p) if rgb is not None else None))
+        return lat, rgb
+
+    def randn(self, seed, count):
+        """The library's seeded N(0,1) stream (sdb_randn): `count` float32 values."""
+        out = np.empty(int(count), np.float32)
+        self.check(self.lib.sdb_randn(self.h, int(seed), int(count), ptr(out)))
+        return out
 
     def img2img(self, context, uncond, scale, n_steps, rgb, strength, mask=None, noise=None, seed=0, latent=True, image=True):
         """rgb [n,8H,8W,3] u8, mask [n,8H,8W] (nonzero = repaint) or None, noise [n,4,H,W] or None (seeded stream).

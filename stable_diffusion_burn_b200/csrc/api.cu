@@ -401,6 +401,35 @@ int sdb_img2img_dev(sdb_ctx* ctx, const uint8_t* d_rgb, const uint8_t* d_mask, c
   API_END
 }
 
+static_assert(SDB_SAMPLER_DDIM == SAMPLER_DDIM && SDB_SAMPLER_DPMPP_2M == SAMPLER_DPMPP_2M, "sampler ids of sdb200.h");
+
+int sdb_sample_ex(sdb_ctx* ctx, const float* context, int n, int L, const float* uncond, int Lu, double guidance_scale,
+                  int n_steps, int sampler, double eta, const float* init_latent, const float* step_noise, uint64_t seed, int H,
+                  int W, float* latent_out, uint8_t* rgb_out) {
+  API_BEGIN(ctx)
+  need_final(c);
+  SDB_CHECK(context && uncond, "null argument");
+  model_sample_ex_host(c, context, n, L, uncond, Lu, guidance_scale, n_steps, sampler, eta, init_latent, step_noise, seed, H, W,
+                       latent_out, rgb_out);
+  API_END
+}
+
+int sdb_sample_ex_dev(sdb_ctx* ctx, const float* d_context, int n, int L, const float* d_uncond, int Lu, double guidance_scale,
+                      int n_steps, int sampler, double eta, const float* d_init_latent, const float* d_step_noise, uint64_t seed,
+                      int H, int W, float* d_latent_out, uint8_t* d_rgb_out, void* stream) {
+  API_BEGIN(ctx)
+  need_final(c);
+  model_sample_ex_dev(c, d_context, n, L, d_uncond, Lu, guidance_scale, n_steps, sampler, eta, d_init_latent, d_step_noise, seed,
+                      H, W, d_latent_out, d_rgb_out, (cudaStream_t)stream);
+  API_END
+}
+
+int sdb_randn(sdb_ctx* ctx, uint64_t seed, int64_t count, float* out) {
+  API_BEGIN(ctx)
+  model_randn_host(c, seed, count, out);
+  API_END
+}
+
 int sdb_clip_forward(sdb_ctx* ctx, const int32_t* tokens, int n, int L, float* out) {
   API_BEGIN(ctx)
   need_final(c);

@@ -1264,18 +1264,91 @@ __device__ __forceinline__ uint32_t mix32(uint32_t x) {
   x ^= x >> 16;
   return x;
 }
+// element i of the seeded N(0,1) stream keyed by (k0, k1): Box-Muller on two hashed uniforms. randn_kernel and
+// cfg_ddim_eta_kernel both draw through this one function, so an in-kernel draw equals randn_launch's output bit for bit.
+__device__ __forceinline__ float randn_at(long long i, uint32_t k0, uint32_t k1) {
+  const uint32_t a = mix32((uint32_t)i ^ k0), b = mix32(((uint32_t)i * 0x9E3779B9u) ^ k1);
+  const float u1 = ((a >> 8) + 1) * (1.0f / 16777216.0f);  // (0,1]
+  const float u2 = (b >> 8) * (1.0f / 16777216.0f);
+  return sqrtf(-2.0f * logf(u1)) * cosf(6.283185307179586f * u2);
+}
+static inline uint32_t randn_key0(uint64_t seed) { return (uint32_t)seed * 2654435761u + 1u; }
+static inline uint32_t randn_key1(uint64_t seed) { return (uint32_t)(seed >> 32) ^ 0x5bd1e995u; }
+
 __global__ void randn_kernel(float* __restrict__ x, long long count, uint32_t k0, uint32_t k1) {
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x) {
-    const uint32_t a = mix32((uint32_t)i ^ k0), b = mix32(((uint32_t)i * 0x9E3779B9u) ^ k1);
-    const float u1 = ((a >> 8) + 1) * (1.0f / 16777216.0f);  // (0,1]
-    const float u2 = (b >> 8) * (1.0f / 16777216.0f);
-    x[i] = sqrtf(-2.0f * logf(u1)) * cosf(6.283185307179586f * u2);
-  }
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x)
+    x[i] = randn_at(i, k0, k1);
 }
 void randn_launch(float* x, long long count, uint64_t seed, cudaStream_t st) {
   int grid = (int)((count + 255) / 256);
   if (grid > 148 * 8) grid = 148 * 8;
-  randn_kernel<<<grid, 256, 0, st>>>(x, count, (uint32_t)seed * 2654435761u + 1u, (uint32_t)(seed >> 32) ^ 0x5bd1e995u);
+  randn_kernel<<<grid, 256, 0, st>>>(x, count, randn_key0(seed), randn_key1(seed));
+  SDB_CUDA(cudaGetLastError());
+}
+
+// ============================================================ selectable samplers (DESIGN.md §7 row f6)
+// Both kernels round once per operation (__f*_rn: no contraction), in the order of oracle/sampler_oracle.py's
+// ddim_update_f32 / dpmpp_2m_update_f32, so a numpy f32 replay of a step matches the device bit for bit.
+__device__ __forceinline__ void cfg_x0_rn(float u, float c, float x, float scale, float sqrt_1m_at, float sqrt_at, float& pred,
+                                          float& x0) {
+  pred = __fadd_rn(u, __fmul_rn(__fsub_rn(c, u), scale));            // stablediffusion/mod.rs:190-191
+  x0 = __fdiv_rn(__fsub_rn(x, __fmul_rn(pred, sqrt_1m_at)), sqrt_at);  // :152
+}
+
+// DDIM with eta > 0: x' = x0*sqrt_anext + pred*dir + sigma*z (mod.rs:153-155 with sigma != 0). z is z_explicit[i], or element i
+// of the seeded stream (k0, k1) when z_explicit is null. sigma == 0 (the last step) reads no noise at all.
+__global__ void cfg_ddim_eta_kernel(const float* __restrict__ eu, const float* __restrict__ ec, float* __restrict__ lat,
+                                    long long count, float scale, float sqrt_1m_at, float sqrt_at, float sqrt_anext, float dir,
+                                    float sigma, const float* __restrict__ z_explicit, uint32_t k0, uint32_t k1) {
+  pdl_enter();
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x) {
+    float pred, x0;
+    cfg_x0_rn(eu[i], ec[i], lat[i], scale, sqrt_1m_at, sqrt_at, pred, x0);
+    float nl = __fadd_rn(__fmul_rn(x0, sqrt_anext), __fmul_rn(pred, dir));
+    if (sigma != 0.0f) nl = __fadd_rn(nl, __fmul_rn(sigma, z_explicit ? z_explicit[i] : randn_at(i, k0, k1)));
+    lat[i] = nl;
+    lat[i + count] = nl;
+  }
+}
+void cfg_ddim_eta_launch(const float* eps_u, const float* eps_c, float* latent, long long count, float scale,
+                         float sqrt_one_minus_at, float sqrt_at, float sqrt_anext, float dir, float sigma, const float* z,
+                         uint64_t z_seed, cudaStream_t st) {
+  int grid = (int)((count + 255) / 256);
+  if (grid > 148 * 8) grid = 148 * 8;
+  launch_k(cfg_ddim_eta_kernel, dim3(grid), dim3(256), 0, st, eps_u, eps_c, latent, count, scale, sqrt_one_minus_at, sqrt_at,
+           sqrt_anext, dir, sigma, z, randn_key0(z_seed), randn_key1(z_seed));
+  SDB_CUDA(cudaGetLastError());
+}
+
+// DPM-Solver++(2M): KIND 0 = first order (D = x0), 1 = second order (D = x0*w0 - hist*w1), 2 = final (x' = x0).
+// x' = x*ratio - D*coef; hist [count] holds x0 of the previous step and receives this step's. The first-order and final
+// variants never read hist (before step 0 it is uninitialised, and 0*NaN is NaN); the final one does not write it either.
+template <int KIND>
+__global__ void cfg_dpmpp2m_kernel(const float* __restrict__ eu, const float* __restrict__ ec, float* __restrict__ lat,
+                                   float* __restrict__ hist, long long count, float scale, float sqrt_1m_at, float sqrt_at,
+                                   float ratio, float coef, float w0, float w1) {
+  pdl_enter();
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x) {
+    const float x = lat[i];
+    float pred, x0;
+    cfg_x0_rn(eu[i], ec[i], x, scale, sqrt_1m_at, sqrt_at, pred, x0);
+    float nl = x0;
+    if (KIND != 2) {
+      const float D = KIND == 0 ? x0 : __fsub_rn(__fmul_rn(x0, w0), __fmul_rn(hist[i], w1));
+      nl = __fsub_rn(__fmul_rn(x, ratio), __fmul_rn(D, coef));
+      hist[i] = x0;
+    }
+    lat[i] = nl;
+    lat[i + count] = nl;
+  }
+}
+void cfg_dpmpp2m_launch(int kind, const float* eps_u, const float* eps_c, float* latent, float* hist, long long count, float scale,
+                        float sqrt_one_minus_at, float sqrt_at, float ratio, float coef, float w0, float w1, cudaStream_t st) {
+  int grid = (int)((count + 255) / 256);
+  if (grid > 148 * 8) grid = 148 * 8;
+  auto k = kind == 0 ? cfg_dpmpp2m_kernel<0> : kind == 1 ? cfg_dpmpp2m_kernel<1> : cfg_dpmpp2m_kernel<2>;
+  launch_k(k, dim3(grid), dim3(256), 0, st, eps_u, eps_c, latent, hist, count, scale, sqrt_one_minus_at, sqrt_at, ratio, coef,
+           w0, w1);
   SDB_CUDA(cudaGetLastError());
 }
 

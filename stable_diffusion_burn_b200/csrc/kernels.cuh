@@ -119,6 +119,16 @@ void quant_conv_slice_launch(const float* x, const float* w, const float* b, int
 void add_vec_launch(const float* a, const float* b, int n, float* y, cudaStream_t st);
 // N(0,1) latents from a Philox-like counter hash (used only when the caller passes no init latent)
 void randn_launch(float* x, long long count, uint64_t seed, cudaStream_t st);
+// ---- selectable samplers (DESIGN.md §7 row f6): CFG + update in one launch, one rounding per operation (no contraction)
+// DDIM with eta > 0: lat' = x0*sqrt_anext + pred*dir + sigma*z; z = z[i], or randn_launch(z_seed)'s element i drawn in-kernel
+// when z is null; sigma == 0 reads no noise. latent holds 2*count floats, written to both halves like cfg_ddim_launch.
+void cfg_ddim_eta_launch(const float* eps_u, const float* eps_c, float* latent, long long count, float scale,
+                         float sqrt_one_minus_at, float sqrt_at, float sqrt_anext, float dir, float sigma, const float* z,
+                         uint64_t z_seed, cudaStream_t st);
+// DPM-Solver++(2M), kind 0 = first order, 1 = second order, 2 = final (lat' = x0): D = x0 | x0*w0 - hist*w1,
+// lat' = x*ratio - D*coef; hist [count] = x0 of the previous step, overwritten with this step's (kinds 0 and 1 only)
+void cfg_dpmpp2m_launch(int kind, const float* eps_u, const float* eps_c, float* latent, float* hist, long long count, float scale,
+                        float sqrt_one_minus_at, float sqrt_at, float ratio, float coef, float w0, float w1, cudaStream_t st);
 
 // ---- row softmax for the 1-head VAE attention: P = softmax(S*scale) rows -> fp16 hi(/lo)
 void softmax_rows_launch(const float* S, long long rows, int cols, float scale, Half2Ptr out, cudaStream_t st);

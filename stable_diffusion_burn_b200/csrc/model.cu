@@ -1084,11 +1084,26 @@ struct SampleStart {
   const uint8_t* m = nullptr;  // [n,H,W] latent mask (0 = keep the known image) or null: no blend
 };
 
+// The update each step applies (DESIGN.md §7 row f6; oracle/sampler_oracle.py states it). The default is the reference's
+// DDIM at eta = 0, which keeps cfg_ddim_kernel and its arguments.
+struct SamplerDesc {
+  int kind = SAMPLER_DDIM;
+  double eta = 0.0;                   // DDIM only
+  const float* step_noise = nullptr;  // [T][n,4,H,W] z of DDIM with eta > 0, or null: the stream of sampler_step_seed(seed, i)
+  uint64_t seed = 0;
+  float* hist = nullptr;              // [n,4,H,W] x0 of the previous step (DPM-Solver++(2M))
+};
+
+uint64_t sampler_step_seed(uint64_t seed, int i) { return seed ^ ((uint64_t)(i + 1) * 0x9E3779B97F4A7C15ull); }
+
+static double half_log_snr(double a) { return std::log(std::sqrt(a) / std::sqrt(1.0 - a)); }
+
 // The DDIM / CFG loop of sample_latent over ts[st.i0:]. Leaves the final latent in the first half of the batch-2n input it
 // returns, with the work arena at the mark after the step state, so the caller can decode from there. The work-arena layout
-// depends on (n, L, Lu, H, W) only: every start index and blend state replays the same cached step graph.
+// depends on (n, L, Lu, H, W) only: every start index, blend state and sampler replays the same cached step graph.
 static float* sample_loop(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale,
-                          int n_steps, const float* d_init_latent, const SampleStart& st, int H, int W) {
+                          int n_steps, const float* d_init_latent, const SampleStart& st, int H, int W,
+                          const SamplerDesc& sd = SamplerDesc{}) {
   Model& m = M(c);
   c.work.reset();
   const int nb = 2 * n;
@@ -1188,6 +1203,7 @@ static float* sample_loop(Ctx& c, const float* d_context, int n, int L, const fl
       m.graphs.push_back(ge);
     }
   }
+  double h_prev = 0.0;  // DPM-Solver++(2M): h of the previous step
   for (size_t i = 0; i < ts.size(); ++i) {
     const int t = ts[i];
     // alphas are read as f32 and widened to f64 (stablediffusion/mod.rs:124-140)
@@ -1202,7 +1218,29 @@ static float* sample_loop(Ctx& c, const float* d_context, int n, int L, const fl
       unet_pass(c, nb, xb, d_tcur, nullptr, Lpad, d_len, H, W, eps, &cs, emb_all);
     }
     KernelScope ks(c, KC_ELEMENTWISE);
-    if (st.m)
+    if (sd.kind == SAMPLER_DPMPP_2M) {
+      // x0 = (x - pred*s_t)/alpha_t; h = lambda_next - lambda_t; x' = (s_next/s_t) x - alpha_next expm1(-h) D, D = x0 at
+      // step 0, (1 + 1/2r) x0 - (1/2r) x0_prev with r = h_prev/h after it; the last step (a_next = 1) returns x0
+      int kind = 2;
+      double ratio = 0, coef = 0, w0 = 0, w1 = 0;
+      if (a_prev < 1.0) {
+        const double h = half_log_snr(a_prev) - half_log_snr(a_t);
+        ratio = std::sqrt(1.0 - a_prev) / std::sqrt(1.0 - a_t), coef = std::sqrt(a_prev) * std::expm1(-h);
+        kind = i == 0 ? 0 : 1;
+        if (kind == 1) w0 = 1.0 + 1.0 / (2.0 * (h_prev / h)), w1 = 1.0 / (2.0 * (h_prev / h));
+        h_prev = h;
+      }
+      cfg_dpmpp2m_launch(kind, eps, eps + le, xb, sd.hist, (long long)le, (float)scale, (float)std::sqrt(1.0 - a_t),
+                         (float)std::sqrt(a_t), (float)ratio, (float)coef, (float)w0, (float)w1, c.stream);
+    } else if (sd.eta > 0.0) {
+      // sigma = eta sqrt((1 - a_next)/(1 - a_t)) sqrt(1 - a_t/a_next), 0 at the last step; x' = x0 sqrt(a_next) +
+      // pred sqrt(1 - a_next - sigma^2) + sigma z (stablediffusion/mod.rs:152-155 with sigma != 0)
+      const int si = st.i0 + (int)i;
+      const double sigma = sd.eta * std::sqrt((1.0 - a_prev) / (1.0 - a_t)) * std::sqrt(1.0 - a_t / a_prev);
+      cfg_ddim_eta_launch(eps, eps + le, xb, (long long)le, (float)scale, (float)std::sqrt(1.0 - a_t), (float)std::sqrt(a_t),
+                          (float)std::sqrt(a_prev), (float)std::sqrt(std::max(0.0, 1.0 - a_prev - sigma * sigma)), (float)sigma,
+                          sd.step_noise ? sd.step_noise + (size_t)si * le : nullptr, sampler_step_seed(sd.seed, si), c.stream);
+    } else if (st.m)
       cfg_ddim_blend_launch(eps, eps + le, xb, (long long)le, (float)scale, (float)std::sqrt(1.0 - a_t), (float)std::sqrt(a_t),
                             (float)std::sqrt(a_prev), (float)std::sqrt(1.0 - a_prev), st.x0, st.eps, st.m, H * W, c.stream);
     else
@@ -1224,6 +1262,71 @@ void model_sample_dev(Ctx& c, const float* d_context, int n, int L, const float*
   const size_t le = (size_t)n * 4 * H * W;
   if (d_latent_out) SDB_CUDA(cudaMemcpyAsync(d_latent_out, xb, le * 4, cudaMemcpyDeviceToDevice, c.stream));
   if (d_rgb) latent_to_image_dev(c, xb, n, H, W, d_rgb);
+}
+
+// ---- selectable samplers (DESIGN.md §7 row f6): DDIM with eta in [0, 1] and DPM-Solver++(2M) on the reference's schedule.
+// The reference fixes sigma = 0 (stablediffusion/mod.rs:119); oracle/sampler_oracle.py states both samplers once.
+static void check_sample_ex_args(const void* latent_out, const void* rgb_out, int n, int L, int Lu, int n_steps, int sampler,
+                                 double eta, const float* step_noise, int H, int W) {
+  SDB_CHECK(sampler == SAMPLER_DDIM || sampler == SAMPLER_DPMPP_2M,
+            "sample_ex: unknown sampler " + std::to_string(sampler) + " (0 = DDIM, 1 = DPM-Solver++(2M))");
+  SDB_CHECK(eta >= 0.0 && eta <= 1.0, "sample_ex: eta must lie in [0, 1]");  // false for NaN
+  SDB_CHECK(sampler == SAMPLER_DDIM || eta == 0.0, "sample_ex: eta applies to DDIM only (DPM-Solver++(2M) takes eta = 0)");
+  SDB_CHECK(!step_noise || (sampler == SAMPLER_DDIM && eta > 0.0), "sample_ex: step_noise is used only by DDIM with eta > 0");
+  SDB_CHECK(latent_out || rgb_out, "sample_ex: latent_out and rgb_out are both null");
+  check_sample_args(n, L, Lu, n_steps, H, W);
+}
+
+void model_sample_ex_dev(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale, int n_steps,
+                         int sampler, double eta, const float* d_init_latent, const float* d_step_noise, uint64_t seed, int H, int W,
+                         float* d_latent_out, uint8_t* d_rgb, cudaStream_t caller) {
+  check_sample_ex_args(d_latent_out, d_rgb, n, L, Lu, n_steps, sampler, eta, d_step_noise, H, W);
+  StreamJoin join(c, caller);
+  const size_t le = (size_t)n * 4 * H * W;
+  // the seeded initial latent and the DPM++ history live in Ctx::state: the work arena keeps the layout of every other sampler
+  if (!d_init_latent) {
+    float* l = (float*)c.state(4, le * 4);
+    KernelScope ks(c, KC_ELEMENTWISE);
+    randn_launch(l, (long long)le, seed, c.stream);  // the stream sdb_sample_latent draws its initial latent from
+    d_init_latent = l;
+  }
+  SamplerDesc sd;
+  sd.kind = sampler, sd.eta = eta, sd.step_noise = d_step_noise, sd.seed = seed;
+  if (sampler == SAMPLER_DPMPP_2M) sd.hist = (float*)c.state(3, le * 4);
+  float* xb = sample_loop(c, d_context, n, L, d_uncond, Lu, scale, n_steps, d_init_latent, SampleStart{}, H, W, sd);
+  if (d_latent_out) SDB_CUDA(cudaMemcpyAsync(d_latent_out, xb, le * 4, cudaMemcpyDeviceToDevice, c.stream));
+  if (d_rgb) latent_to_image_dev(c, xb, n, H, W, d_rgb);
+}
+
+void model_sample_ex_host(Ctx& c, const float* context, int n, int L, const float* uncond, int Lu, double scale, int n_steps,
+                          int sampler, double eta, const float* init_latent, const float* step_noise, uint64_t seed, int H, int W,
+                          float* latent_out, uint8_t* rgb) {
+  check_sample_ex_args(latent_out, rgb, n, L, Lu, n_steps, sampler, eta, step_noise, H, W);
+  const size_t le = (size_t)n * 4 * H * W, ce = (size_t)n * L * 768, ue = (size_t)Lu * 768, re = (size_t)n * 3 * 64 * H * W;
+  const size_t ne = step_noise ? ddim_timesteps(n_steps).size() * le : 0;
+  float* d_c = (float*)c.io(0, ce * 4);
+  float* d_u = (float*)c.io(1, ue * 4);
+  float* d_l = init_latent ? (float*)c.io(2, le * 4) : nullptr;
+  float* d_z = step_noise ? (float*)c.io(3, ne * 4) : nullptr;
+  float* d_lo = latent_out ? (float*)c.io(4, le * 4) : nullptr;
+  uint8_t* d_r = rgb ? (uint8_t*)c.io(5, re) : nullptr;
+  SDB_CUDA(cudaMemcpyAsync(d_c, context, ce * 4, cudaMemcpyHostToDevice, c.stream));
+  SDB_CUDA(cudaMemcpyAsync(d_u, uncond, ue * 4, cudaMemcpyHostToDevice, c.stream));
+  if (init_latent) SDB_CUDA(cudaMemcpyAsync(d_l, init_latent, le * 4, cudaMemcpyHostToDevice, c.stream));
+  if (step_noise) SDB_CUDA(cudaMemcpyAsync(d_z, step_noise, ne * 4, cudaMemcpyHostToDevice, c.stream));
+  model_sample_ex_dev(c, d_c, n, L, d_u, Lu, scale, n_steps, sampler, eta, d_l, d_z, seed, H, W, d_lo, d_r, c.stream);
+  if (latent_out) SDB_CUDA(cudaMemcpyAsync(latent_out, d_lo, le * 4, cudaMemcpyDeviceToHost, c.stream));
+  if (rgb) SDB_CUDA(cudaMemcpyAsync(rgb, d_r, re, cudaMemcpyDeviceToHost, c.stream));
+  SDB_CUDA(cudaStreamSynchronize(c.stream));
+}
+
+void model_randn_host(Ctx& c, uint64_t seed, int64_t count, float* out) {
+  SDB_CHECK(count >= 0 && (out || count == 0), "randn: count must be >= 0 and out non-null");
+  if (count == 0) return;
+  float* d = (float*)c.io(0, (size_t)count * 4);
+  randn_launch(d, (long long)count, seed, c.stream);
+  SDB_CUDA(cudaMemcpyAsync(out, d, (size_t)count * 4, cudaMemcpyDeviceToHost, c.stream));
+  SDB_CUDA(cudaStreamSynchronize(c.stream));
 }
 
 // ---- img2img (SDEdit) and latent-blend inpainting (DESIGN.md §7 row f5). The reference has no img2img: this is the standard

@@ -31,6 +31,19 @@ void model_img2img_dev(Ctx& c, const uint8_t* d_rgb_in, const uint8_t* d_mask, c
 void model_img2img_host(Ctx& c, const uint8_t* rgb_in, const uint8_t* mask, const float* context, int n, int L,
                         const float* uncond, int Lu, double scale, int n_steps, double strength, const float* noise, uint64_t seed,
                         int H, int W, float* latent_out, uint8_t* rgb);
+// text-to-image with a selectable sampler (DESIGN.md §7 row f6): sampler SAMPLER_DDIM (eta in [0,1]; eta = 0 is
+// model_sample_dev exactly) or SAMPLER_DPMPP_2M (eta = 0). step_noise [T][n,4,H,W] (DDIM with eta > 0 only) or null: slice i is
+// then drawn in-kernel from the randn_launch stream keyed by sampler_step_seed(seed, i). init_latent null: randn_launch(seed).
+enum SamplerKind : int { SAMPLER_DDIM = 0, SAMPLER_DPMPP_2M = 1 };
+uint64_t sampler_step_seed(uint64_t seed, int i);
+void model_sample_ex_dev(Ctx& c, const float* d_context, int n, int L, const float* d_uncond, int Lu, double scale, int n_steps,
+                         int sampler, double eta, const float* d_init_latent, const float* d_step_noise, uint64_t seed, int H, int W,
+                         float* d_latent_out, uint8_t* d_rgb, cudaStream_t caller);
+void model_sample_ex_host(Ctx& c, const float* context, int n, int L, const float* uncond, int Lu, double scale, int n_steps,
+                          int sampler, double eta, const float* init_latent, const float* step_noise, uint64_t seed, int H, int W,
+                          float* latent_out, uint8_t* rgb);
+// the N(0,1) stream of randn_launch keyed by seed, count values into host memory
+void model_randn_host(Ctx& c, uint64_t seed, int64_t count, float* out);
 void model_forward_diffuser_dev(Ctx& c, const float* d_latent, int t, const float* d_context, int n, int L, const float* d_uncond,
                                 int Lu, double scale, int H, int W, float* d_pred, float* d_u, float* d_c, cudaStream_t caller);
 void model_forward_diffuser_host(Ctx& c, const float* latent, int t, const float* context, int n, int L, const float* uncond,

@@ -149,8 +149,10 @@ struct Ctx {
     size_t cap = 0;
   } iobuf[8];
   void* io(int slot, size_t bytes);
-  // grow-only device state of the img2img sampler (encoded image, noise, latent mask): it must survive the work-arena reset
-  // between the encoder and the step loop, and it is never one of the host wrappers' staging slots
+  // grow-only device state of the samplers: slots 0-2 img2img (encoded image, noise, latent mask), which must survive the
+  // work-arena reset between the encoder and the step loop; slot 3 the DPM-Solver++(2M) history x0_{i-1} and slot 4 the seeded
+  // initial latent of sdb_sample_ex_dev, kept out of the work arena so that every sampler replays the same step graph. None is
+  // ever one of the host wrappers' staging slots.
   IoBuf statebuf[8];
   void* state(int slot, size_t bytes);
   void io_destroy();  // frees iobuf and statebuf

@@ -94,17 +94,32 @@ class StableDiffusion:
         return self
 
     # ---- hot path
+    # sampler = "ddim" (eta in [0,1]; the reference's sampler is eta = 0) or "dpmpp_2m" (DPM-Solver++(2M), eta = 0); step_noise
+    # [T,n,4,H/8,W/8] is the per-step noise of DDIM with eta > 0 (None: the seeded stream). DESIGN.md §7 row f6. The defaults
+    # take the reference's own entry points.
     def sample_image(self, context, unconditional_context, unconditional_guidance_scale: float, n_steps: int,
-                     init_latent=None, seed: int = 0, height: int = 512, width: int = 512):
+                     init_latent=None, seed: int = 0, height: int = 512, width: int = 512, sampler: str = "ddim",
+                     eta: float = 0.0, step_noise=None):
         """-> list of n flat uint8 arrays of H*W*3 (HWC RGB), like the reference's Vec<Vec<u8>>."""
-        rgb = self.ctx.sample_image(context, unconditional_context, unconditional_guidance_scale, n_steps,
-                                    init_latent=init_latent, seed=seed, H=height // 8, W=width // 8)
+        if sampler == "ddim" and eta == 0.0 and step_noise is None:
+            rgb = self.ctx.sample_image(context, unconditional_context, unconditional_guidance_scale, n_steps,
+                                        init_latent=init_latent, seed=seed, H=height // 8, W=width // 8)
+        else:
+            _, rgb = self.ctx.sample_ex(context, unconditional_context, unconditional_guidance_scale, n_steps, sampler=sampler,
+                                        eta=eta, init_latent=init_latent, step_noise=step_noise, seed=seed, H=height // 8,
+                                        W=width // 8, latent=False, image=True)
         return [rgb[i].reshape(-1) for i in range(rgb.shape[0])]
 
     def sample_latent(self, context, unconditional_context, unconditional_guidance_scale: float, n_steps: int,
-                      init_latent=None, seed: int = 0, height: int = 512, width: int = 512) -> np.ndarray:
-        return self.ctx.sample_latent(context, unconditional_context, unconditional_guidance_scale, n_steps,
-                                      init_latent=init_latent, seed=seed, H=height // 8, W=width // 8)
+                      init_latent=None, seed: int = 0, height: int = 512, width: int = 512, sampler: str = "ddim",
+                      eta: float = 0.0, step_noise=None) -> np.ndarray:
+        if sampler == "ddim" and eta == 0.0 and step_noise is None:
+            return self.ctx.sample_latent(context, unconditional_context, unconditional_guidance_scale, n_steps,
+                                          init_latent=init_latent, seed=seed, H=height // 8, W=width // 8)
+        lat, _ = self.ctx.sample_ex(context, unconditional_context, unconditional_guidance_scale, n_steps, sampler=sampler,
+                                    eta=eta, init_latent=init_latent, step_noise=step_noise, seed=seed, H=height // 8,
+                                    W=width // 8)
+        return lat
 
     def img2img(self, context, unconditional_context, unconditional_guidance_scale: float, n_steps: int, image, strength: float,
                 mask=None, noise=None, seed: int = 0):
